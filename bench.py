@@ -2,7 +2,7 @@
 """bench.py — superpoints/s (fwd+bwd) of the hierarchical superpoint-graph
 attention + pooling stack on the BASELINE.json cfg-2 workload.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Own arm (default): one process per GPU (torchrun for N>1), every rank owns one
 cfg-2 scene (scene-shard data parallelism, weak scaling), one flat NCCL gradient
@@ -79,6 +79,7 @@ BENCH_CONFIGS['tiny'] = dict(levels=[2_000, 400, 80], no_ffn=True, scaling='weak
                              metric=METRIC, workload=f"tiny: 2k/400/80 superpoints (test only); {_MODEL}")
 LEVELS = BENCH_CONFIGS['cfg2']['levels']
 WORKLOAD = BENCH_CONFIGS['cfg2']['workload']
+DUMP_BYTES = 60 << 20   # --dump-outputs: 64 MB in all, with room for the .npy headers
 
 
 def model_kwargs(S=None, no_ffn=True):
@@ -302,6 +303,26 @@ def rank_micro_batches(cfg_name, rank, world):
     raise ValueError(cfg_name)
 
 
+def write_outputs(out_dir, loss, logits, grad, budget=DUMP_BYTES):
+    """--dump-outputs: what one step of the own arm computed, as float32 .npy files in `out_dir`:
+    loss.npy (cross-entropy of every micro-batch of this rank), logits.npy (the head's output on
+    the level-1 rows of those micro-batches, in order) and grad.npy (the flat gradient buffer the
+    optimizer stepped with).  Where all of it would exceed `budget` bytes, logits.npy holds a
+    fixed, seeded sample of the rows, ascending, and logits_rows.npy (float64) their row numbers."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    loss, logits, grad = (t.detach().float().cpu().numpy() for t in (loss, logits, grad))
+    if loss.nbytes + logits.nbytes + grad.nbytes > budget:
+        room = (budget - loss.nbytes - grad.nbytes) // (logits[0].nbytes + 8)
+        assert room > 0, f'loss and gradient alone exceed the {budget}-byte budget'
+        rows = torch.randperm(logits.shape[0], generator=torch.Generator().manual_seed(0))[:room]
+        rows = rows.sort().values.numpy()
+        logits = logits[rows]
+        np.save(os.path.join(out_dir, 'logits_rows.npy'), rows.astype(np.float64))
+    for name, a in (('loss', loss), ('logits', logits), ('grad', grad)):
+        np.save(os.path.join(out_dir, f'{name}.npy'), a)
+
+
 def device_transforms(S, nag):
     nag = S.transforms.NodeSize()(nag)
     # csr_order: edges emitted grouped by source (the model is invariant to edge order), so the
@@ -384,6 +405,18 @@ def run_own(args):
     flat = FlatGradients(params)
     opt = torch.optim.AdamW(params, lr=1e-3, weight_decay=1e-4, fused=True,
                             capturable=not args.no_graph)
+    init_params = [p.detach().clone() for p in params]
+
+    def reset_training_state():
+        """Every step of the resident phase trains from the seeded initial parameters and a
+        fresh AdamW state.  The gradient reductions add with float atomics, so a chain of
+        optimizer steps would drift apart from run to run; this way the same arguments give
+        the same inputs to every step and the same outputs up to rounding."""
+        with torch.no_grad():
+            torch._foreach_copy_(params, init_params)
+            state = [t for p in params for t in opt.state[p].values() if torch.is_tensor(t)]
+            if state:
+                torch._foreach_zero_(state)
 
     # this rank's share of one step: a list of micro-batches (host side, pinned)
     micro, shard_info = rank_micro_batches(cfg_name, rank, world)
@@ -398,10 +431,18 @@ def run_own(args):
     # accumulated gradient is the gradient of the mean loss of the whole step
     loss_scale = [m[3] / sp_total * world for m in micro]   # all_reduce divides by world
 
+    last = {}   # micro-batch -> (loss, logits) of the latest step, for --dump-outputs
+
     def fwd_bwd(nag, labels, i_mb):
         flat.release()
         out = net(nag)
-        loss = torch.nn.functional.cross_entropy(head(out), labels)
+        logits = head(out)
+        loss = torch.nn.functional.cross_entropy(logits, labels)
+        if args.dump_outputs:
+            last[i_mb] = (loss, logits)
+        # the backward reuses the logits' memory; holding them through it costs ~0.7 % of a
+        # cfg-2 step, so only a dumping run does
+        del logits
         (loss * loss_scale[i_mb] if (n_mb > 1 or world > 1) else loss).backward()
         flat.collect(accumulate=i_mb > 0)
         return loss
@@ -465,6 +506,7 @@ def run_own(args):
 
     def eager_step():
         loss = None
+        reset_training_state()
         for i in range(n_mb):
             restore(i)
             loss = fwd_bwd(resident[i][0], resident[i][1], i)
@@ -490,8 +532,10 @@ def run_own(args):
                     return fwd_bwd(resident[i][0], resident[i][1], i)
                 graphs.append(Graphed(body, pool=pool))
             g_opt = Graphed(lambda: opt.step(), pool=pool)
+            g_reset = Graphed(reset_training_state, pool=pool)   # after g_opt made the state
 
             def run_resident():   # noqa: F811
+                g_reset()
                 for gph in graphs:
                     loss = gph()
                 flat.all_reduce()
@@ -510,6 +554,10 @@ def run_own(args):
         time.sleep(0.3)
     ms, t0, t1 = timed(run_resident, args.steps)
     clocks = sampler.stop(t0, t1) if sampler else None
+    if args.dump_outputs and rank == 0:
+        # a CUDA graph replays into the tensors it captured, so `last` holds the last timed step
+        write_outputs(args.dump_outputs, torch.stack([last[i][0] for i in range(n_mb)]),
+                      torch.cat([last[i][1] for i in range(n_mb)]), flat.flat)
     # count my launches per step and time my kernels with CUDA events (eager steps: the
     # same kernels on the same inputs; events cannot be read back from a graph replay)
     for _ in range(2):
@@ -705,7 +753,11 @@ def run_own(args):
                                "TMA (csrc/gemm_umma.cu)",
                      "csr": "graph CSR cached across steps in `value` (amortised, SURVEY §8d); "
                             "rebuilt every step in `e2e`; on-the-fly edges emitted in CSR order "
-                            "(OnTheFlyHorizontalEdgeFeatures(csr_order=True))"},
+                            "(OnTheFlyHorizontalEdgeFeatures(csr_order=True))",
+                     "training_state": "every step of `value` starts from the seeded initial "
+                                       "parameters and a fresh AdamW state (one captured copy + "
+                                       "zero): the same arguments give the same outputs up to "
+                                       "the rounding of one backward"},
             "clocks": clocks,
             "e2e": {"value": round(e2e_value, 1), "unit": UNIT,
                     "ms_per_step": round(ms_e2e / e2e_steps, 4),
@@ -913,12 +965,17 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-graph', action='store_true', help='eager launches, no CUDA graphs')
     ap.add_argument('--kernels-out', default=None, help='write the full per-kernel timing table (JSON)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the loss, logits and gradient of the last timed step as .npy '
+                         'files in DIR (own arm)')
     ap.add_argument('--model', default='baseline', choices=['baseline', 'shipped64', 'shipped128'],
                     help="'baseline': the BASELINE.json model (C=128, 4 heads); 'shipped64' / "
                          "'shipped128': the head layout of the shipped configs (16 heads, C = 64 "
                          "as S3DIS / DALES, C = 128 as KITTI-360) on the same graphs — not a "
                          "BASELINE configuration, reported with `config.model_variant`")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes what the own arm computed; the reference arm has none')
     if args.model != 'baseline':
         global DIM, HEADS
         DIM, HEADS = (64, 16) if args.model == 'shipped64' else (128, 16)

@@ -2,6 +2,9 @@
 and a REAL partition as test data — tests/golden/demo_nag.pt is the reference's demo room
 (notebooks/demo_nag_v3.h5: 41 568 points, 1 192 / 501 / 166 superpoints) as read by
 superpoint_transformer_b200.io (tests/make_demo_fixture.py).  CPU only."""
+import hashlib
+import json
+import lzma
 import os
 
 import pytest
@@ -15,9 +18,9 @@ from superpoint_transformer_b200.transforms import (SampleSubNodes, SampleSegmen
                                                    SampleKHopSubgraphs)
 
 from test_select import assert_level_equal, levels_of, to_product, oracle_primitives  # noqa
+from make_demo_fixture import FIXTURE_H5_XZ, FIXTURE_H5_JSON, hole_tensor
 
 FIXTURE = os.path.join(os.path.dirname(__file__), 'golden', 'demo_nag.pt')
-DEMO_H5 = '/root/reference/notebooks/demo_nag_v3.h5'
 
 
 def as_long(level):
@@ -34,6 +37,23 @@ def as_long(level):
 def demo():
     raw = torch.load(FIXTURE, weights_only=False)
     return {'start': raw['start'], 'levels': [as_long(lv) for lv in raw['levels']]}
+
+
+@pytest.fixture(scope='module')
+def demo_h5(tmp_path_factory):
+    """The reference's demo file, byte for byte: its committed copy with the holes refilled from
+    demo_nag.pt (tests/make_demo_fixture.py), checked against the original's SHA-256."""
+    with open(FIXTURE_H5_JSON) as fh:
+        manifest = json.load(fh)
+    with open(FIXTURE_H5_XZ, 'rb') as fh:
+        buf = bytearray(lzma.decompress(fh.read()))
+    raw = torch.load(FIXTURE, weights_only=False)
+    for name, addr, nbytes in manifest['holes']:
+        buf[addr:addr + nbytes] = hole_tensor(raw, name).numpy().tobytes()
+    assert hashlib.sha256(buf).hexdigest() == manifest['sha256']
+    path = tmp_path_factory.mktemp('demo') / 'demo_nag_v3.h5'
+    path.write_bytes(buf)
+    return str(path)
 
 
 def test_demo_partition_is_a_consistent_hierarchy(demo):
@@ -56,33 +76,31 @@ def test_demo_partition_is_a_consistent_hierarchy(demo):
     assert 'edge_index' not in levels[0] and levels[0]['rgb'].dtype == torch.uint8
 
 
-def test_reader_and_loaders_reproduce_the_fixture():
-    if not os.path.isfile(DEMO_H5):
-        pytest.skip('reference demo file not mounted')
+def test_reader_and_loaders_reproduce_the_fixture(demo_h5):
     from superpoint_transformer_b200.io import H5File, load_nag
     raw = torch.load(FIXTURE, weights_only=False)
-    with H5File(DEMO_H5) as f:
+    with H5File(demo_h5) as f:
         assert f.keys() == ['level_0', 'level_1', 'level_2', 'level_3']
         assert int(f.attrs['start_i_level']) == 0
         assert f['level_1/_not_indexable_'].read() == ['sub', 'edge_attr', 'edge_index']
         assert f['level_0/pos'].shape == (41568, 3) and str(f['level_0/pos'].dtype) == 'float32'
         assert f['level_2/_cluster_/sub'].keys() == ['is_index_value', 'pointers', 'value_0']
-    nag = NAG.load(DEMO_H5)
+    nag = NAG.load(demo_h5)
     assert isinstance(nag, NAG) and nag.num_points == [41568, 1192, 501, 166]
     for got, want in zip(levels_of(nag), raw['levels']):
         assert_level_equal(got, want, 'fixture')
     # integers widened, colours as floats, a level range, a key subset
-    part = NAG.load(DEMO_H5, low=1, high=2, keys=['pos', 'super_index', 'sub', 'rgb'],
+    part = NAG.load(demo_h5, low=1, high=2, keys=['pos', 'super_index', 'sub', 'rgb'],
                     non_fp_to_long=True)
     assert part.start_i_level == 1 and part.num_levels == 2 and sorted(part[1].keys) == \
         ['pos', 'sub', 'super_index']
     assert part[1].super_index.dtype == torch.int64 and part[2].sub.points.dtype == torch.int64
-    full = load_nag(DEMO_H5, non_fp_to_long=True, rgb_to_float=True)
+    full = load_nag(demo_h5, non_fp_to_long=True, rgb_to_float=True)
     assert full[0].rgb.dtype == torch.float32 and float(full[0].rgb.max()) <= 1.0
     assert torch.equal((full[0].rgb * 255).round().byte(), nag[0].rgb)
     with pytest.raises(NotImplementedError):
-        NAG.load(DEMO_H5, idx=torch.arange(10))
-    level = Data.load(H5File(DEMO_H5)['level_3'], non_fp_to_long=True)
+        NAG.load(demo_h5, idx=torch.arange(10))
+    level = Data.load(H5File(demo_h5)['level_3'], non_fp_to_long=True)
     assert level.num_nodes == 166 and isinstance(level.sub, Cluster)
 
 
@@ -121,14 +139,12 @@ def test_save_load_round_trip(demo, tmp_path):
     assert level.num_nodes == 501 and torch.equal(level.sub.points, cases['demo'][2].sub.points)
 
 
-def test_written_file_has_the_reference_files_structure(tmp_path):
-    """In the build container: saving the loaded demo partition gives the reference file's own
-    inventory (names, shapes, stored dtypes) and the same header messages byte for byte."""
-    if not os.path.isfile(DEMO_H5):
-        pytest.skip('reference demo file not mounted')
+def test_written_file_has_the_reference_files_structure(demo_h5, tmp_path):
+    """Saving the loaded demo partition gives the reference file's own inventory (names,
+    shapes, stored dtypes) and the same header messages byte for byte."""
     from superpoint_transformer_b200.io import H5File
     out = str(tmp_path / 'again.h5')
-    NAG.load(DEMO_H5).save(out)
+    NAG.load(demo_h5).save(out)
 
     def inventory(g, path=''):
         items = {}
@@ -140,7 +156,7 @@ def test_written_file_has_the_reference_files_structure(tmp_path):
                 items[f'{path}/{k}'] = (o.shape, str(o.dtype))
         return items
 
-    ref, mine = H5File(DEMO_H5), H5File(out)
+    ref, mine = H5File(demo_h5), H5File(out)
     assert inventory(ref) == inventory(mine) and len(inventory(mine)) == 63
     assert ref._r.buf[8:24] == mine._r.buf[8:24]                    # superblock parameters
 

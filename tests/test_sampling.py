@@ -189,46 +189,6 @@ def test_host_logic_subgraph_sampling_matches_reference(gold, nags, oracle_primi
         SampleKHopSubgraphs(i_level=7)(nag)
 
 
-def test_reference_loader_regenerates_sampling_vectors(gold, nags):
-    """In the build container: the committed vectors are what the reference's own
-    src/transforms/sampling.py gives under the recorded torch seeds."""
-    from oracle import reference_data as R
-    if not R.available():
-        pytest.skip('reference sources not mounted')
-    from oracle.make_golden_select import to_reference, level_dict
-    ns = R.load_data()
-
-    def same(res, want):
-        for j, b in enumerate(want):
-            assert_level_equal(level_dict(ns, res[j]), b, f'regen level {j}')
-
-    for case in gold['segments'][::2]:
-        spec = nags[case['nag']]
-        torch.manual_seed(case['seed'])
-        same(ns.SampleSegments(ratio=case['ratio'], by_size=case['by_size'],
-                               by_class=case['by_class'])(
-            to_reference(ns, spec['levels'], spec['start'])), case['out'])
-    for case in gold['restrict'][::2]:
-        spec = nags[case['nag']]
-        torch.manual_seed(case['seed'])
-        same(ns.NAGRestrictSize(level=case['level'], num_nodes=case['num_nodes'],
-                                num_edges=case['num_edges'])(
-            to_reference(ns, spec['levels'], spec['start'])), case['out'])
-    for case in gold['subgraphs'][::3]:
-        spec = nags[case['nag']]
-        nag = to_reference(ns, spec['levels'], spec['start'])
-        if case['batches'] is not None:
-            for i, b in enumerate(case['batches']):
-                nag[i].batch = b.clone()
-        cls = ns.SampleKHopSubgraphs if case['kind'] == 'khop' else ns.SampleRadiusSubgraphs
-        torch.manual_seed(case['seed'])
-        same(cls(disjoint=False, **case['kw'])(nag), case['out'])
-    case = gold['sparse'][1]
-    _, ptr = ns.sparse_sample(case['idx'], n_max=case['n_max'], n_min=case['n_min'],
-                              mask=case['mask'], return_pointers=True)
-    assert torch.equal(ptr, case['ptr_samples'])
-
-
 def test_sampling_without_label_histograms(nags, oracle_primitives):
     """Levels without `y` (the synthetic benchmark partitions): by_class has nothing to use and
     the weights stay uniform (+ size term), as with the reference's `Data.y is None`."""
